@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — HNSW k-NN queries/sec on synthetic f32 vectors (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 A step = one pass of the hot path (batched hnsw_knn) over one batch of B queries.
 
@@ -82,7 +82,14 @@ def parse():
     ap.add_argument("--watchdog-s", type=int, default=int(os.environ.get("COZO_BENCH_WATCHDOG_S", 840)),
                     help="end the process (rc 3) if the run has not finished after this many seconds: a wedged kernel "
                          "must not hold the GPU box until the caller's limit (0 = off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32 / float64), so that two "
+                         "builds can be compared output for output on the same seeded inputs")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if a.workload in WORKLOADS:
         rows, batch, k, tile, scaling = WORKLOADS[a.workload]
         world = int(os.environ.get("WORLD_SIZE", 1))
@@ -222,6 +229,26 @@ def mem_available_bytes() -> int:
     except OSError:
         pass
     return 0
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array (all share their first axis).  Integer ids are written as float64,
+    which holds them exactly.  When the arrays exceed 64 MB in all, the same seeded sample of rows is kept of each,
+    and the sampled row numbers go to DIR/sample_rows.npy."""
+    arrays = {k: np.asarray(v, np.float32 if np.asarray(v).dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(v.nbytes for v in arrays.values()) // n
+    if n * row_bytes > DUMP_BYTES:
+        keep = (DUMP_BYTES - 4096) // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(0x5EED0005).choice(n, keep, replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["sample_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
 
 
 def recall_rows(a_ids, b_ids, k):
@@ -369,6 +396,8 @@ def run_pagerank(a):
         kms.append(ms)
     t_end = time.perf_counter()
     clocks = sampler.stop(t_start, t_end)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"scores": scores})
     tot_ms = sum(kms)
     value = m * iters * a.steps / (tot_ms / 1e3)
     bytes_iter = 8 * m + 20 * n
@@ -534,6 +563,9 @@ def main():
     if world > 1:
         dist.barrier()
     clocks = sampler.stop(t_start, t_end)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"ids": (ids if grp is None else out_i).cpu().numpy(),
+                                      "distances": (dd if grp is None else out_d).cpu().numpy()})
     total_ms = e_all0.elapsed_time(e_all1)
     if world > 1:
         t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
