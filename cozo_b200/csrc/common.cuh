@@ -116,4 +116,12 @@ __device__ __forceinline__ float4 ldg_nc_f4(const float4* p) {
 }
 #endif
 
+// Key order of every sorted distance list (search beams, per-shard top-k lists), the reference's OrderedFloat:
+// NaN sorts after every number, +inf included, and equal keys keep arrival order.  A raw `<=` is false for NaN, so
+// a NaN key (0/0 of a zero-norm Cosine row) would go first and break the sorted prefix behind it.
+template <typename T>
+__device__ __forceinline__ bool precedes(T a, T b) {
+  return a < b || (isnan(b) && !isnan(a));
+}
+
 }  // namespace cozo

@@ -442,12 +442,14 @@ __device__ __forceinline__ void build_link_body(const HnswDev& g, const BuildDev
       u_d[deg + lane] = ad;
     }
     __syncwarp();
-    for (uint32_t j = lane; j < nc; j += 32) {  // rank sort by (distance, position)
+    // rank sort by (distance, position).  The order must be total for the ranks to be a permutation: with raw
+    // compares every NaN distance (a zero-norm Cosine row) got rank 0 and slots of s_id were left unwritten.
+    for (uint32_t j = lane; j < nc; j += 32) {
       float dj = u_d[j];
       uint32_t rank = 0;
       for (uint32_t x = 0; x < nc; ++x) {
         float dx = u_d[x];
-        rank += (dx < dj) || (dx == dj && x < j);
+        rank += precedes(dx, dj) || (!precedes(dj, dx) && x < j);
       }
       s_id[rank] = u_id[j];
       s_d[rank] = dj;

@@ -142,12 +142,12 @@ __device__ __forceinline__ float dist_ldg1(const float4 (&q)[NV], const float4* 
 }
 
 // found_nn.push + pop-if-over-ef (hnsw.rs:577-580) on the sorted array.
-// Precondition: len < ef || d < fd[len-1].  Equal keys keep arrival order.
+// Precondition: len < ef || d < fd[len-1].  Equal keys keep arrival order; NaN keys sort last (`precedes`).
 __device__ __forceinline__ void sorted_insert(WarpCtx& w, uint32_t ef, float d, uint32_t id, int lane) {
   uint32_t pos = 0;
   for (uint32_t base = 0; base < w.len; base += 32) {
     uint32_t i = base + lane;
-    bool le = (i < w.len) && (w.fd[i] <= d);
+    bool le = (i < w.len) && !precedes(d, w.fd[i]);
     uint32_t bal = __ballot_sync(0xffffffffu, le);
     pos += __popc(bal);
     if (bal != 0xffffffffu) break;

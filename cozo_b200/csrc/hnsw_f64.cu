@@ -63,12 +63,12 @@ __device__ __forceinline__ double dist64(const double* q, const double* __restri
   return 1.0 - a / sqrt(qnorm * b);
 }
 
-// found_nn.push + pop-if-over-ef (hnsw.rs:577-580) on the sorted array; equal keys keep arrival order
+// found_nn.push + pop-if-over-ef (hnsw.rs:577-580) on the sorted array; equal keys keep arrival order, NaN sorts last
 __device__ __forceinline__ void sorted_insert64(WarpCtx& w, double* fd, uint32_t ef, double d, uint32_t id, int lane) {
   uint32_t pos = 0;
   for (uint32_t base = 0; base < w.len; base += 32) {
     uint32_t i = base + lane;
-    bool le = (i < w.len) && (fd[i] <= d);
+    bool le = (i < w.len) && !precedes(d, fd[i]);
     uint32_t bal = __ballot_sync(0xffffffffu, le);
     pos += __popc(bal);
     if (bal != 0xffffffffu) break;

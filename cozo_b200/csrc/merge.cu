@@ -31,7 +31,8 @@ __global__ void __launch_bounds__(128) topk_merge_kernel(const float* __restrict
         size_t at = ((size_t)s * B + q) * k + pos[j];
         float d = dist[at];
         uint32_t id = ids[at];
-        if (id != NONE && (d < my_d || (d == my_d && s < my_shard))) {
+        // (dist, shard) order with NaN last: a NaN head is taken once every finite head is out
+        if (id != NONE && (my_shard == NONE || precedes(d, my_d) || (!precedes(my_d, d) && s < my_shard))) {
           my_d = d;
           my_shard = s;
           my_pos = pos[j];
@@ -41,14 +42,14 @@ __global__ void __launch_bounds__(128) topk_merge_kernel(const float* __restrict
   };
   refresh();
   for (uint32_t r = 0; r < k; ++r) {
-    // warp argmin on (dist, shard)
+    // warp argmin on (dist, shard); NONE = this lane's shards are exhausted
     float bd = my_d;
     uint32_t bs = my_shard;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
       float od = __shfl_xor_sync(0xffffffffu, bd, o);
       uint32_t os = __shfl_xor_sync(0xffffffffu, bs, o);
-      if (od < bd || (od == bd && os < bs)) {
+      if (os != NONE && (bs == NONE || precedes(od, bd) || (!precedes(bd, od) && os < bs))) {
         bd = od;
         bs = os;
       }

@@ -105,9 +105,12 @@ def _pytest_on_emu(lib, args, timeout):
 
 def test_gpu_test_files_on_the_emulated_library(emu_lib):
     """the host-layer GPU tests (FixedRule / HnswSearchRA mirrors over the C ABI: PageRank, Dijkstra incl. keep_ties, Yen,
-    centralities, clustering, index build / write-back / put / rm, device filter) and the quick graph tests, unchanged,
-    with the binding pointed at libcozo_gpu_emu.so"""
-    out = _pytest_on_emu(emu_lib, ["-m", "gpu", "tests/test_host_gpu.py", "tests/test_graph_gpu.py", "-k", "not air_routes and not 17-5"], 2400)
+    centralities, clustering, index build / write-back / put / rm, device filter), the quick graph tests and the NaN
+    ordering of zero-norm Cosine rows, unchanged, with the binding pointed at libcozo_gpu_emu.so"""
+    out = _pytest_on_emu(emu_lib, ["-m", "gpu", "tests/test_host_gpu.py", "tests/test_graph_gpu.py",
+                                   "tests/test_search_widths_gpu.py::test_nan_cosine_exhaustive",
+                                   "tests/test_search_widths_gpu.py::test_nan_non_exhaustive_built_index",
+                                   "-k", "not air_routes and not 17-5"], 2400)
     assert " passed" in out and "failed" not in out
 
 
@@ -115,4 +118,5 @@ def test_gpu_test_files_on_the_emulated_library(emu_lib):
 def test_all_gpu_test_files_on_the_emulated_library(emu_lib):
     """every -m gpu / gpu_unverified test that does not need torch CUDA tensors, several GPUs or a million vectors"""
     _pytest_on_emu(emu_lib, ["-m", "gpu or gpu_unverified", "-p", "no:timeout", "tests/test_graph_gpu.py", "tests/test_hnsw_gpu.py",
-                             "tests/test_host_gpu.py", "tests/test_unverified_gpu.py", "-k", "not search_dev_and_merge"], 4 * 3600)
+                             "tests/test_host_gpu.py", "tests/test_unverified_gpu.py", "tests/test_search_widths_gpu.py",
+                             "-k", "not search_dev_and_merge"], 4 * 3600)
